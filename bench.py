@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """VQACL train-step throughput on B200 (BASELINE.json metric: train samples/s, VL-T5 base, 36 RoIs).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one synthetic batch of configs[1]: VLT5VQA.train_step (forward with the SI
 prototype update/retrieval) + loss.backward() + clip_grad_norm_(5) + HF AdamW, B = 320 per GPU, 36 x 2048 RoI features,
@@ -17,6 +17,13 @@ per GPU, weak scaling, gradients averaged over NCCL from inside backward.
           configs[0] (B = 8), rank 0 only
 `--impl reference` times that CPU path alone (the reference is pure PyTorch and cannot be imported here — SURVEY.md H3 —
 so the oracle port is the reference arm).
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller, as DIR/<name>.npy (float32, or float64 for
+integers): train mode the loss, the prototype-retrieval indices, the encoder attention mask, the logits and encoder hidden
+states of a fixed seeded sample of batch rows, the SI prototype banks, and a fixed seeded sample of every parameter after
+the optimizer step; decode mode the generated token ids. Inputs, weights and dropout seeds depend only on the arguments,
+so two builds can be compared output for output (weight gradients accumulate with fp32 atomics, so the comparison needs
+a tolerance, not bit equality).
 """
 import argparse
 import json
@@ -28,9 +35,35 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 
 FLOP_PER_SAMPLE_STEP = 37.79e9          # SURVEY.md §8(d): forward 12.634 GFLOP x 3 minus the unneeded VisEmbed dX (T = 5, S = 56)
 METRIC = "VQACL train samples/s (VL-T5 base, 36 RoIs)"
+DUMP_ROWS = 16                          # --dump-outputs: batch rows kept of the [B, ...] float outputs (logits alone are 206 MB)
+DUMP_PARAM_ELEMS = 1024                 # --dump-outputs: elements kept of every parameter
+DUMP_LIMIT = 64 << 20
+
+
+def dump_rows(B):
+    """The fixed, seeded sample of batch rows --dump-outputs keeps."""
+    import torch
+    return torch.randperm(B, generator=torch.Generator().manual_seed(0))[:min(B, DUMP_ROWS)].sort().values
+
+
+def write_dump(out_dir, arrays):
+    """arrays: name -> tensor; written as out_dir/<name>.npy, integers as float64 (exact), floats as float32."""
+    import numpy as np
+    import torch
+    host = {}
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        host[name] = (t.double() if not t.is_floating_point() or t.dtype == torch.float64 else t.float()).numpy()
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def step_flops(N=36, L=20, T=5, d=768, f=3072, V=32200, F=2048, Le=12, Ld=12):
@@ -224,8 +257,17 @@ def run_native(args):
         devb.append({k: v.to(dev) for k, v in b.items()})
     h2d = sum(v.numel() * v.element_size() for v in host[0].values())
 
-    def step(batch, read_loss):
+    dumped = {}
+    rows = dump_rows(B).to(dev) if args.dump_outputs else None
+
+    def step(batch, read_loss, keep=False):
         r = model.train_step(batch, task, 0.5, 0.3)
+        if keep:
+            # device copies taken as train_step returns: the returned tensors are views of workspaces later kernels reuse
+            dumped.update(loss=r["loss"].detach().clone(), max_idx_Q=r["max_idx_Q"].clone(), max_idx_V=r["max_idx_V"].clone(),
+                          encoder_attention_mask=r["encoder_attention_mask"].clone(), sample_rows=rows,
+                          logits_sample=r["logits"].index_select(0, rows),
+                          encoder_hidden_states_sample=r["encoder_hidden_states"].index_select(0, rows))
         r["loss"].backward()
         opt.step(max_grad_norm=5.0)
         sched.step()
@@ -236,7 +278,7 @@ def run_native(args):
 
     prefetcher = {}
 
-    def timed(batches, steps, warmup, read_loss, prefetch=False):
+    def timed(batches, steps, warmup, read_loss, prefetch=False, keep_last=False):
         if prefetch:
             prefetcher["p"] = V.BatchPrefetcher(None, dev)
             prefetcher["p"].loader = [batches[i % pool] for i in range(max(warmup, 4))]
@@ -258,7 +300,7 @@ def run_native(args):
                 step(b, read_loss)
         else:
             for i in range(steps):
-                step(batches[i % pool], read_loss)
+                step(batches[i % pool], read_loss, keep=keep_last and i == steps - 1)
         model.param_sync()          # an overlapped optimizer tail of the last step belongs to the timed region
         e1.record()
         if world > 1:
@@ -275,8 +317,15 @@ def run_native(args):
     clocks = ClockSampler(local)
     if rank == 0:
         clocks.start()
-    ms, launches = timed(devb, args.steps, warm, False)
+    ms, launches = timed(devb, args.steps, warm, False, keep_last=bool(args.dump_outputs))
     ck = clocks.stop() if rank == 0 else None
+    if args.dump_outputs:
+        g = torch.Generator().manual_seed(0)
+        params = [v.detach().reshape(-1)[torch.randint(0, v.numel(), (min(v.numel(), DUMP_PARAM_ELEMS),), generator=g).to(v.device)]
+                  for v in model.state_dict().values() if v.is_floating_point()]
+        dumped.update(Q_prototype=model.Q_prototype, V_prototype=model.V_prototype, params_sample=torch.cat([p.float() for p in params]))
+        if rank == 0:
+            write_dump(args.dump_outputs, dumped)
     ms_e2e, _ = timed(host, args.steps, 2, True, prefetch=True)
     # the literal drop-in call: pinned CPU batch straight into train_step, whose own .to(device) copies it on the compute stream
     ms_dropin, _ = timed(host, args.steps, 2, True, prefetch=False)
@@ -356,7 +405,9 @@ def run_decode(args):
     devb = [{k: v.to(dev) for k, v in b.items()} for b in host]
     h2d = sum(host[0][k].numel() * host[0][k].element_size() for k in ("vis_feats", "boxes", "input_ids"))
 
-    def timed(batches, steps, warmup, to_host):
+    dumped = {}
+
+    def timed(batches, steps, warmup, to_host, keep_last=False):
         ntok = 0
         for i in range(warmup):
             model.test_step(batches[i % pool])
@@ -368,6 +419,8 @@ def run_decode(args):
         e0.record()
         for i in range(steps):
             t = model.test_step(batches[i % pool])["token_ids"]
+            if keep_last and i == steps - 1:
+                dumped["token_ids"] = t.clone()
             ntok += t.shape[1] - 1
             if to_host:
                 t = t.cpu()                        # the answers leave the device (tokenizer.batch_decode runs on the host)
@@ -386,8 +439,10 @@ def run_decode(args):
     clocks = ClockSampler(local)
     if rank == 0:
         clocks.start()
-    ms, launches, ntok = timed(devb, args.steps, warm, False)
+    ms, launches, ntok = timed(devb, args.steps, warm, False, keep_last=bool(args.dump_outputs))
     ck = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        write_dump(args.dump_outputs, dumped)
     ms_e2e, _, _ = timed(host, args.steps, 2, True)
     if rank == 0:
         c = cfg
@@ -432,8 +487,14 @@ def main():
     ap.add_argument("--no-kernel-roofline", action="store_true")
     ap.add_argument("--no-overlap-optimizer", action="store_true",
                     help="run clip+AdamW on the main stream instead of overlapping it with the next step's forward")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the native implementation")
         # torchrun exports OMP_NUM_THREADS=1; the CPU arm uses every host core (set before torch is imported)
         os.environ["OMP_NUM_THREADS"] = str(os.cpu_count() or 1)
         os.environ.pop("MKL_NUM_THREADS", None)

@@ -4,6 +4,7 @@ import os
 import pytest
 import torch
 
+from golden_fixtures import assert_close_to_sample, load_prototype_path, load_vlt5_forward
 from helpers import O
 
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -21,7 +22,7 @@ def test_visual_embedding_matches_reference():
 
 
 def test_prototype_state_machine_matches_reference():
-    d = torch.load(os.path.join(G, "prototype_path.pt"))
+    d = load_prototype_path()
     bank = O.PrototypeBank()
     for st in d["steps"]:
         h = st["hidden"].float()
@@ -58,7 +59,7 @@ def test_full_forward_glue_matches_reference():
     mask construction (a3), SI path in place (a9-a13), shift-right, cross mask with the two prototype rows attendable,
     decoder, x d^-1/2, tied LM head, CE(reduction='none') (a7, a8, a14), over four consecutive calls on one model, then one
     step through the reference's VLT5VQA.train_step text (a1)."""
-    d = torch.load(os.path.join(G, "vlt5_forward.pt"))
+    d = load_vlt5_forward()
     cfg = O.VLT5Config(dropout_rate=0.0, **d["cfg"])
     om = O.VLT5VQA(cfg).eval()
     missing, unexpected = om.load_state_dict(d["state"], strict=False)
@@ -75,7 +76,7 @@ def test_full_forward_glue_matches_reference():
             kw = dict(cate_labels=c["cate_labels"], ques_labels=c["ques_labels"], proto_update=True, task_id=c["task"],
                       alpha=d["alpha"], beta=d["beta"]) if c["proto_update"] else {}
             out = om(c["input_ids"], c["vis_feats"], c["boxes"], c["labels"], **kw)
-        torch.testing.assert_close(out["encoder_hidden_states"], c["encoder_hidden_states"], rtol=1e-5, atol=1e-5)
+        assert_close_to_sample(out["encoder_hidden_states"], c["encoder_hidden_states"], rtol=1e-5, atol=1e-5)
         assert torch.equal(out["encoder_attention_mask"], c["encoder_attention_mask"])
         torch.testing.assert_close(out["logits"], c["logits"], rtol=1e-4, atol=1e-4)
         torch.testing.assert_close(out["loss"], c["loss"], rtol=1e-4, atol=1e-5)
@@ -89,7 +90,7 @@ def test_full_forward_glue_matches_reference():
                             t["task"], d["alpha"], d["beta"], 3, 1000)
     assert set(t["keys"]) <= set(res.keys()) and tuple(res["BL"]) == tuple(t["BL"])
     torch.testing.assert_close(res["loss"], t["loss"], rtol=1e-5, atol=1e-6)
-    torch.testing.assert_close(res["encoder_hidden_states"], t["encoder_hidden_states"], rtol=1e-5, atol=1e-5)
+    assert_close_to_sample(res["encoder_hidden_states"], t["encoder_hidden_states"], rtol=1e-5, atol=1e-5)
     assert torch.equal(res["encoder_attention_mask"], t["encoder_attention_mask"])
     torch.testing.assert_close(om.bank.Q_prototype, t["Q_prototype"], rtol=1e-5, atol=1e-6)
     torch.testing.assert_close(om.bank.V_prototype, t["V_prototype"], rtol=1e-5, atol=1e-6)

@@ -8,6 +8,7 @@ import torch
 import torch.nn.functional as F
 
 import cabi
+from golden_fixtures import load_prototype_path
 from helpers import O, cos, rel_err
 
 pytestmark = pytest.mark.gpu
@@ -114,7 +115,7 @@ def test_prototype_kernels_match_reference_fixture_bit_exact_bookkeeping():
     """calculate_current_prototype / update_prototype / cosine_similarity_multi through the C-ABI against the fixture
     produced by executing the reference's own source (tools/gen_golden.py): counts, slot routing and argmax indices are
     compared bit-exact, prototype values to fp32 round-off (summation order differs)."""
-    d = torch.load(os.path.join(G, "prototype_path.pt"))
+    d = load_prototype_path()
     Q = torch.zeros(10, 768, device=DEV)
     Vp = torch.zeros(80, 768, device=DEV)
     numQ = torch.zeros(10, device=DEV)

@@ -8,7 +8,8 @@ hot path that do not depend on the 4.2.1 internals can be lifted out of the file
     (the only edit: the hard-coded torch.device('cuda') string at :504 is evaluated on CPU)
   * the loss tail of VLT5VQA.train_step         VL-T5/src/vqa_model.py:46-54
 The fixtures hold seeded inputs and the reference's outputs; tests/test_golden.py checks the oracle against them on CPU
-and tests/test_gpu_ops.py checks the CUDA path. Nothing is copied into the repo except these tensors. (tools/gen_golden_forward.py does the same for the glue of a whole
+and tests/test_gpu_ops.py checks the CUDA path. Nothing is copied into the repo except these tensors (prototype_path.pt
+in the compact layout of tests/golden_fixtures.py: seeded inputs are regenerated, not stored). (tools/gen_golden_forward.py does the same for the glue of a whole
 call: JointEncoder.forward + VLT5.forward.)
 
     python tools/gen_golden.py [/root/reference]
@@ -23,6 +24,8 @@ import torch.nn as nn
 
 REF = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+sys.path.insert(0, os.path.dirname(OUT))
+from golden_fixtures import pack_prototype_path, prototype_inputs  # noqa: E402  (seeded inputs + the stored layout)
 SRC = os.path.join(REF, "VL-T5", "src", "modeling_t5_our.py")
 SRC_VQA = os.path.join(REF, "VL-T5", "src", "vqa_model.py")
 
@@ -78,38 +81,21 @@ def main():
     # ---------------------------------------------------------------- prototype functions
     m = VLT5.__new__(VLT5)          # no __init__: only the dict/attribute state the three methods touch
     m.Q_task_mem_proto, m.Q_task_cur_proto = {}, {}
-    g = torch.Generator().manual_seed(202)
-    steps = []
-    Bp, Sp = 8, 26          # 20 'text' + 6 'visual' rows: the split index 20 is hard-coded in the reference (:381)
     # task 0: two steps; task 2: three steps (first / first-mem / EMA); task 5: one step. alpha .5 beta .3
-    schedule = [(0, 0), (0, 1), (2, 2), (2, 3), (2, 4), (5, 5)]
-    for task, sd in schedule:
-        hidden = torch.randn(Bp, Sp, 768, generator=g).bfloat16().float()   # bf16-representable -> stored compactly
-        if sd == 3:
-            hidden[:, :, :] *= 0.5
-        ql = torch.zeros(Bp, 10)
-        qcls = torch.randint(0, task + 1, (Bp,), generator=g) if task > 0 else torch.zeros(Bp, dtype=torch.long)
-        ql[torch.arange(Bp), qcls] = 1
-        cl = torch.zeros(Bp, 80)
-        cl[torch.arange(Bp), torch.randint(0, 80, (Bp,), generator=g)] = 1
+    steps, P, x = prototype_inputs()
+    for st in steps:
+        hidden, ql, cl, task = st["hidden"], st["ques_labels"], st["cate_labels"], st["task"]
         curQ, numQ = m.calculate_current_prototype(hidden[:, :20, :], ql)
         curV, numV = m.calculate_current_prototype(hidden[:, 20:, :], cl)
         m.update_prototype(curQ, curV, numQ, numV, task, 0.5, 0.3)
         rq, iq, _ = m.cosine_similarity_multi(m.Q_prototype, torch.mean(hidden[:, :20, :], dim=1), ql)
         rv, iv, _ = m.cosine_similarity_multi(m.V_prototype, torch.mean(hidden[:, 20:, :], dim=1), cl)
-        steps.append(dict(task=task, hidden=hidden.bfloat16(), ques_labels=ql, cate_labels=cl, curQ=curQ.clone(), curV=curV.clone(),
-                          numQ=numQ.clone(), numV=numV.clone(), Q_prototype=m.Q_prototype.clone(),
-                          V_prototype=m.V_prototype.clone(), Q_num=m.Q_prototype_num.clone(), V_num=m.V_prototype_num.clone(),
-                          retr_Q=rq.clone(), idx_Q=iq.clone(), retr_V=rv.clone(), idx_V=iv.clone()))
+        st.update(curQ=curQ.clone(), curV=curV.clone(), numQ=numQ.clone(), numV=numV.clone(), Q_prototype=m.Q_prototype.clone(),
+                  V_prototype=m.V_prototype.clone(), Q_num=m.Q_prototype_num.clone(), V_num=m.V_prototype_num.clone(),
+                  retr_Q=rq.clone(), idx_Q=iq.clone(), retr_V=rv.clone(), idx_V=iv.clone())
     # eval-time retrieval without labels, with an all-zero row present (tie-break / zero-row behaviour, SURVEY.md a12)
-    P = torch.randn(10, 768, generator=g)
-    P[0] = 0
-    P[7] = 0
-    x = torch.randn(9, 768, generator=g)
-    x[3] = -P[1] * 2          # negative similarity to every real row except maybe others
     rq, iq, _ = m.cosine_similarity_multi(P, x)
-    torch.save(dict(steps=steps, alpha=0.5, beta=0.3, eval_P=P, eval_x=x, eval_retr=rq, eval_idx=iq),
-               os.path.join(OUT, "prototype_path.pt"))
+    torch.save(pack_prototype_path(steps, 0.5, 0.3, P, x, rq, iq), os.path.join(OUT, "prototype_path.pt"))
 
     # ---------------------------------------------------------------- loss tail (vqa_model.py:46-54)
     text = open(SRC_VQA).read().splitlines()

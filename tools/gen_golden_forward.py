@@ -30,6 +30,7 @@ import torch.nn.functional as F
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 from gen_golden import lift  # noqa: E402
+from golden_fixtures import pack_vlt5_forward  # noqa: E402  (gen_golden puts tests/ on the path)
 
 REF = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
@@ -194,8 +195,8 @@ def main():
             state["decoder." + k] = v.clone()
     os.makedirs(OUT, exist_ok=True)
     path = os.path.join(OUT, "vlt5_forward.pt")
-    torch.save(dict(calls=calls, train_call=train_call, state=state, cfg=dict(vocab_size=VOCAB, d_model=D, d_kv=DKV, d_ff=FF, num_heads=H, feat_dim=FEAT,
-                                                       num_layers=1, num_decoder_layers=1), alpha=0.5, beta=0.3), path)
+    torch.save(pack_vlt5_forward(calls, train_call, state, dict(vocab_size=VOCAB, d_model=D, d_kv=DKV, d_ff=FF, num_heads=H, feat_dim=FEAT,
+                                                                num_layers=1, num_decoder_layers=1), 0.5, 0.3), path)
     print(path, os.path.getsize(path))
 
 
