@@ -175,6 +175,13 @@ int vqacl_gemm_bf16(const void* A, int lda, int a_mn_major, const void* B, int l
 int vqacl_gemm_bf16_ex(const void* A, int lda, int a_mn_major, const void* B, int ldb, int b_mn_major, void* C, int ldc,
                        const void* R, int ldr, int M, int N, int K, int epi, float alpha, int splits, int force_bn,
                        uint32_t drop_thr16, float inv_keep, uint32_t drop_key, void* stream);
+/* split-K with one fp32 slab per split (the decoder FFN-out form: a consumer adds the slabs in a fixed order, deterministic
+ * unlike the atomic epilogue): slab s = C + s * split_stride ([M, N], pitch ldc, split_stride >= M * ldc) receives
+ * alpha * A[:, Ks] B[:, Ks]^T over split s's range Ks of 64-deep k-blocks. The requested split count is clamped to the number
+ * of k-blocks and rounded so that no split is empty; *n_slabs receives the count used, and slabs past it are not written.   */
+int vqacl_gemm_bf16_slabs(const void* A, int lda, int a_mn_major, const void* B, int ldb, int b_mn_major, float* C, int ldc,
+                          long long split_stride, int M, int N, int K, float alpha, int splits, int force_bn, int* n_slabs,
+                          void* stream);
 /* nn.Linear + residual add + the T5LayerNorm that opens the NEXT sub-layer in one launch (HF T5LayerSelfAttention / T5LayerFF
  * followed by the next layer_norm): C(f32)[M,768] = R + A[M,K] B[768,K]^T; n_out(bf16) = C * rsqrt(mean(C^2) + eps) * norm_w.       */
 int vqacl_gemm_resid_rmsnorm(const void* A, int lda, const void* B, int ldb, float* C, const float* R, int M, int K,

@@ -33,6 +33,11 @@ def _L():
                                          c_int, F, c_int, c_int, ctypes.c_uint32, F, ctypes.c_uint32, c_void_p]
         L.vqacl_gemm_resid_rmsnorm.argtypes = [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, F, c_void_p, c_void_p]
         L.vqacl_visual_embed_fused.argtypes = [c_void_p, c_void_p, c_int] + [c_void_p] * 8 + [c_int] * 5 + [F, c_void_p, c_void_p, c_void_p]
+        L.vqacl_gemm_bf16_slabs.argtypes = [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_int, c_int64, c_int, c_int, c_int, F,
+                                            c_int, c_int, ctypes.POINTER(c_int), c_void_p]
+        L.vqacl_set_gemm_sm_limit.argtypes = [c_int]
+        L.vqacl_set_gemm_dynamic_schedule.argtypes = [c_int]
+        L.vqacl_launch_count.restype = ctypes.c_longlong
         L._ops_declared = True
     return L
 
@@ -197,3 +202,26 @@ def gemm_grouped_mn(As, Bs, Cs, epi=3, alpha=1.0):
                                        IP(*[b.stride(0) for b in Bs]), VP(*[c.data_ptr() for c in Cs]), IP(*[c.stride(0) for c in Cs]),
                                        IP(*[a.shape[1] for a in As]), IP(*[b.shape[1] for b in Bs]), K, epi, ctypes.c_float(alpha), cur_stream()))
     return Cs
+
+
+def gemm_slabs(A, a_mn, B, b_mn, C, M, N, K, split_stride, alpha=1.0, splits=1, bn=0):
+    """Split-K with one fp32 slab per split: slab s = C.view(-1)[s * split_stride:] with pitch C.stride(0). Returns the number of
+    slabs the GEMM wrote."""
+    n = c_int(-1)
+    check(_L().vqacl_gemm_bf16_slabs(ptr(A), A.stride(0), int(a_mn), ptr(B), B.stride(0), int(b_mn), ptr(C), C.stride(0), split_stride,
+                                     M, N, K, alpha, splits, bn, ctypes.byref(n), cur_stream()))
+    return n.value
+
+
+def set_gemm_sm_limit(n):
+    """Process-wide: SMs the persistent GEMMs may occupy (0 = all; odd values are rounded down to even)."""
+    check(_L().vqacl_set_gemm_sm_limit(int(n)))
+
+
+def set_gemm_dynamic_schedule(on):
+    """Process-wide: atomic-counter tile schedule of the CTA-pair kernel instead of the static round robin."""
+    check(_L().vqacl_set_gemm_dynamic_schedule(int(bool(on))))
+
+
+def launch_count():
+    return int(_L().vqacl_launch_count())

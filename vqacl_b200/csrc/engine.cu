@@ -462,8 +462,7 @@ static int decoder_forward(Engine& e, const vqacl_batch* b, cudaStream_t st) {
   // unlike an atomic meeting point. VQACL_DEC_FFN_SPLITS=1 restores the single-pass residual epilogue.
   static const int fsplit_req = [] { const char* ev = getenv("VQACL_DEC_FFN_SPLITS"); const int v = ev ? atoi(ev) : 3; return v >= 1 && v <= 3 ? v : 3; }();
   // the slab count the GEMM will really use (gemm_bf16 never leaves a K slice empty): the norm kernel must add exactly those
-  const int ffn_kb = (f + 63) / 64, ffn_per = (ffn_kb + fsplit_req - 1) / fsplit_req;
-  const int fsplit = (ffn_kb + ffn_per - 1) / ffn_per;
+  const int fsplit = gemm_split_count(f, fsplit_req);
   auto ffn_out_pending = [&](RmsFwdArgs& r, int l_prev) {     // make r's norm consume the slabs of layer l_prev's FFN-out GEMM
     r.parts = w.t_parts; r.n_parts = fsplit; r.part_stride = (long long)Md * d;
     r.resid = w.y[3 * l_prev + 2]; r.x_out = w.y[3 * l_prev + 3]; r.resid_drop = e.drop(site_dec(l_prev, 5));

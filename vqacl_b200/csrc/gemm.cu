@@ -322,10 +322,26 @@ static int dispatch_major(const GemmOperand& A, const GemmOperand& B, const Gemm
   VQ_CHECK(false, "gemm: A MN-major with B K-major is not instantiated");
 }
 
+int gemm_split_count(int K, int splits) {
+  const int kblocks = (K + GEMM_BK - 1) / GEMM_BK;
+  if (splits < 1) splits = 1;
+  if (splits > kblocks) splits = kblocks;
+  const int per = (kblocks + splits - 1) / splits;   // k-blocks per split, rounded so that no split is empty
+  return (kblocks + per - 1) / per;
+}
+
 int gemm_bf16(const GemmOperand& A, const GemmOperand& B, GemmArgs args, int force_bn, cudaStream_t stream) {
   VQ_CHECK(args.M > 0 && args.N > 0 && args.K > 0, "gemm: empty problem %d x %d x %d", args.M, args.N, args.K);
   VQ_CHECK(args.N % 8 == 0, "gemm: N=%d must be a multiple of 8", args.N);
-  VQ_CHECK(args.ldc % 8 == 0, "gemm: ldc=%d must be a multiple of 8", args.ldc);
+  VQ_CHECK(args.ldc % 8 == 0 && args.ldc >= (args.epi == EPI_ARGMAX ? 1 : args.N), "gemm: ldc=%d must be a multiple of 8 and >= N=%d",
+           args.ldc, args.N);
+  // the epilogue stores (and the residual epilogue loads) 16-byte vectors; the mask epilogues access one u32 word per 32 columns
+  VQ_CHECK(args.C && (args.epi == EPI_ARGMAX || (reinterpret_cast<uintptr_t>(args.C) & 15) == 0), "gemm: C %p is not 16-byte aligned", args.C);
+  VQ_CHECK(args.epi != EPI_RESID_F32 || (args.R && (reinterpret_cast<uintptr_t>(args.R) & 15) == 0 && args.ldr % 4 == 0 && args.ldr >= args.N),
+           "gemm: the residual epilogue needs a 16-byte aligned R with a pitch that is a multiple of 4 and >= N");
+  VQ_CHECK(args.epi != EPI_RELUBWD_BF16 || args.R, "gemm: the ReLU-backward epilogue needs the sign bitmask R");
+  VQ_CHECK((args.epi != EPI_RELU_BF16 && args.epi != EPI_RELUBWD_BF16) || !args.R || args.ldr >= (args.N + 31) / 32,
+           "gemm: the sign bitmask needs ldr >= %d words", (args.N + 31) / 32);
   if (args.splits < 1) args.splits = 1;
   VQ_CHECK(args.splits == 1 || args.epi == EPI_ATOMIC_F32 || (args.epi == EPI_F32 && args.split_stride >= (long long)args.M * args.ldc),
            "gemm: split-K needs the atomic epilogue, or the fp32 one with a slab stride");
@@ -345,12 +361,7 @@ int gemm_bf16(const GemmOperand& A, const GemmOperand& B, GemmArgs args, int for
     VQ_CHECK(args.C && args.R && args.ldc >= slots && args.ldr >= slots, "gemm: argmax partial buffers need %d slots per row", slots);
   }
   const int kblocks = (args.K + GEMM_BK - 1) / GEMM_BK;
-  if (args.splits > kblocks) args.splits = kblocks;
-  // make sure no split is empty
-  {
-    int per = (kblocks + args.splits - 1) / args.splits;
-    args.splits = (kblocks + per - 1) / per;
-  }
+  args.splits = gemm_split_count(args.K, args.splits);
   int bn = force_bn;
   if (bn == 0) {
     // pick the tile shape that minimises waves x per-tile MMA time. Cycles per 64-deep k-block:
@@ -413,6 +424,24 @@ extern "C" int vqacl_gemm_bf16(const void* A, int lda, int a_mn_major, const voi
   g.alpha = alpha;
   g.splits = splits;
   return vq::gemm_bf16(a, b, g, force_bn, reinterpret_cast<cudaStream_t>(stream));
+}
+
+// split-K with one fp32 slab per split (the decoder FFN-out form, epilogue 5 with a slab stride)
+extern "C" int vqacl_gemm_bf16_slabs(const void* A, int lda, int a_mn_major, const void* B, int ldb, int b_mn_major, float* C, int ldc,
+                                     long long split_stride, int M, int N, int K, float alpha, int splits, int force_bn, int* n_slabs,
+                                     void* stream) {
+  VQ_CHECK(n_slabs != nullptr, "gemm_slabs: n_slabs is null");
+  vq::GemmOperand a{A, lda, a_mn_major != 0}, b{B, ldb, b_mn_major != 0};
+  vq::GemmArgs g{};
+  g.epi = vq::EPI_F32;
+  g.M = M; g.N = N; g.K = K;
+  g.C = C; g.ldc = ldc;
+  g.alpha = alpha;
+  g.splits = splits;
+  g.split_stride = split_stride;
+  if (vq::gemm_bf16(a, b, g, force_bn, reinterpret_cast<cudaStream_t>(stream))) return 1;
+  *n_slabs = vq::gemm_split_count(K, splits);
+  return 0;
 }
 
 // same with the epilogue dropout exposed (epi 1 and 2): drop_thr16 = round(p * 65536) (0 disables), drop_key = the per-launch

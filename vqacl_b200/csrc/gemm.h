@@ -12,6 +12,9 @@ struct GemmOperand {
 
 // C[M,N] (+)= A[M,K] * B[N,K]^T with the epilogue in args.epi. force_bn = 0 picks the N tile by occupancy.
 int gemm_bf16(const GemmOperand& A, const GemmOperand& B, GemmArgs args, int force_bn, cudaStream_t stream);
+// split-K factor gemm_bf16 really uses for a request of `splits` over K: clamped to the 64-deep k-blocks and rounded so that
+// no split is empty (a consumer of the split_stride slabs must add exactly this many)
+int gemm_split_count(int K, int splits);
 // n <= GEMM_GROUP_MAX independent weight-gradient problems C_i[M_i, N_i] += A_i[M_i, K] * B_i[N_i, K]^T (both operands MN-major,
 // shared K) as ONE launch of the CTA-pair kernel; epi = EPI_ATOMIC_F32 (accumulate) or EPI_F32 (store)
 struct GemmGroupProblem {
