@@ -201,6 +201,19 @@ int vqacl_attention_bwd(const void* q, const void* k, const void* v, int ldq, in
                         const float* rel_table, const int32_t* rel_bucket, int rel_mode, int Lt, const float* keymask, int causal,
                         float* d_rel_table, const void* o_saved /* forward output (pitch ldo) or NULL: enables the key-split
                         backward for Sq <= 16 < Sk */, void* stream);
+/* same with the dropout on the probabilities (drop_thr16 = round(p * 65536), inv_keep = 1 / (1 - p), drop_key = per-launch
+ * 32-bit key; drop_thr16 = 0 disables it) and, forward only, the KV-cache decode form: element strides between batch entries
+ * (0 = densely packed, Sq * ld resp. Sk * ld), and q_off = absolute position of query row 0 (0 <= q_off, q_off + Sq <= 64).
+ * lse may be NULL in the forward.                                                                                             */
+int vqacl_attention_fwd_ex(const void* q, const void* k, const void* v, int ldq, int ldk, int ldv, void* o, int ldo, float* lse,
+                           int B, int H, int Sq, int Sk, const float* rel_table, const int32_t* rel_bucket, int rel_mode, int Lt,
+                           const float* keymask, int causal, uint32_t drop_thr16, float inv_keep, uint32_t drop_key,
+                           int64_t q_bstride, int64_t k_bstride, int64_t v_bstride, int64_t o_bstride, int q_off, void* stream);
+int vqacl_attention_bwd_ex(const void* q, const void* k, const void* v, int ldq, int ldk, int ldv, const void* dO, int ldo,
+                           const float* lse, void* dq, void* dk, void* dv, int lddq, int lddk, int lddv, int B, int H, int Sq, int Sk,
+                           const float* rel_table, const int32_t* rel_bucket, int rel_mode, int Lt, const float* keymask, int causal,
+                           float* d_rel_table, const void* o_saved, uint32_t drop_thr16, float inv_keep, uint32_t drop_key,
+                           void* stream);
 /* SI prototype path (modeling_t5_our.py:583-615): token means of hidden[:, :split] / hidden[:, split:] (:585-588,601-605) */
 int vqacl_proto_means(const float* h, int B, int S, int split, float* meanQ, float* meanV, void* stream);
 /* VLT5.calculate_current_prototype (modeling_t5_our.py:500-511)                                                              */

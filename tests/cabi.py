@@ -17,6 +17,9 @@ def _L():
         L.vqacl_attention_fwd.argtypes = [c_void_p] * 3 + [c_int] * 3 + [c_void_p, c_int, c_void_p] + [c_int] * 4 + [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p]
         L.vqacl_attention_bwd.argtypes = ([c_void_p] * 3 + [c_int] * 3 + [c_void_p, c_int, c_void_p] + [c_void_p] * 3 + [c_int] * 3 + [c_int] * 4 +
                                           [c_void_p, c_void_p, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p])
+        L.vqacl_attention_fwd_ex.argtypes = (L.vqacl_attention_fwd.argtypes[:-1] + [ctypes.c_uint32, F, ctypes.c_uint32] + [c_int64] * 4 +
+                                             [c_int, c_void_p])
+        L.vqacl_attention_bwd_ex.argtypes = L.vqacl_attention_bwd.argtypes[:-1] + [ctypes.c_uint32, F, ctypes.c_uint32, c_void_p]
         L.vqacl_proto_means.argtypes = [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]
         L.vqacl_proto_scatter_mean.argtypes = [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]
         L.vqacl_proto_update.argtypes = [c_void_p] * 8 + [c_int] * 5 + [F, F, c_void_p]
@@ -75,6 +78,29 @@ def attention_bwd(q, k, v, dO, lse, B, H, Sq, Sk, rel_table=None, rel_bucket=Non
                                    ptr(dq), ptr(dk), ptr(dv), dq.stride(0), dk.stride(0), dv.stride(0), B, H, Sq, Sk, ptr(rel_table),
                                    ptr(rel_bucket), rel_mode, Lt, ptr(keymask), causal, ptr(dtab), ptr(o_saved), cur_stream()))
     return dq, dk, dv, dtab
+
+
+def _pitch(t, ld=None):
+    """row pitch of a 2-D operand: stride(0) unless given; 0 for a missing (NULL) operand"""
+    return ld if ld is not None else 0 if t is None else t.stride(0)
+
+
+def attention_fwd_ex(q, k, v, o, lse, B, H, Sq, Sk, rel_table=None, rel_bucket=None, rel_mode=0, Lt=0, keymask=None, causal=0,
+                     drop=(0, 1.0, 0), bstrides=(0, 0, 0, 0), q_off=0, ld=(None, None, None, None)):
+    """vqacl_attention_fwd_ex into caller-provided o (and lse, or None). Pointers are the tensors' first elements; the row pitches
+    are their stride(0) unless given in ld = (ldq, ldk, ldv, ldo). drop = (thr16, inv_keep, key)."""
+    check(_L().vqacl_attention_fwd_ex(ptr(q), ptr(k), ptr(v), _pitch(q, ld[0]), _pitch(k, ld[1]), _pitch(v, ld[2]), ptr(o), _pitch(o, ld[3]),
+                                      ptr(lse), B, H, Sq, Sk, ptr(rel_table), ptr(rel_bucket), rel_mode, Lt, ptr(keymask), causal,
+                                      int(drop[0]), float(drop[1]), int(drop[2]), *[int(x) for x in bstrides], q_off, cur_stream()))
+
+
+def attention_bwd_ex(q, k, v, dO, lse, dq, dk, dv, d_rel_table, B, H, Sq, Sk, rel_table=None, rel_bucket=None, rel_mode=0, Lt=0,
+                     keymask=None, causal=0, o_saved=None, drop=(0, 1.0, 0)):
+    """vqacl_attention_bwd_ex into caller-provided dq / dk / dv (row pitches = their stride(0)); d_rel_table is accumulated into."""
+    check(_L().vqacl_attention_bwd_ex(ptr(q), ptr(k), ptr(v), _pitch(q), _pitch(k), _pitch(v), ptr(dO), _pitch(dO), ptr(lse),
+                                      ptr(dq), ptr(dk), ptr(dv), _pitch(dq), _pitch(dk), _pitch(dv), B, H, Sq, Sk, ptr(rel_table),
+                                      ptr(rel_bucket), rel_mode, Lt, ptr(keymask), causal, ptr(d_rel_table), ptr(o_saved),
+                                      int(drop[0]), float(drop[1]), int(drop[2]), cur_stream()))
 
 
 def proto_means(h, split):
@@ -158,7 +184,12 @@ def gemm_dropout(A, B, C, R, M, N, K, epi, thr16, inv_keep, key, bn=0):
 
 def dropout_scale_host(M, N, thr16, inv_keep, key, device):
     """Host restatement of vq_dropout_pair (csrc/common.cuh): scale (0 or inv_keep) of every element of an [M, N] matrix."""
-    idx = torch.arange(M * N, device=device, dtype=torch.int64).view(M, N)
+    return dropout_scale_idx(torch.arange(M * N, device=device, dtype=torch.int64).view(M, N), thr16, inv_keep, key)
+
+
+def dropout_scale_idx(idx, thr16, inv_keep, key):
+    """Scale (0 or inv_keep) of the elements with int64 element indices `idx`: pair idx >> 1 is hashed with the 32-bit key, the
+    low 16 bits of the hash decide the even element of the pair and the high 16 bits the odd one."""
     m32 = 0xFFFFFFFF
     x = ((idx >> 1) * 0x9E3779B1 + key) & m32
     x = x ^ (x >> 16)

@@ -216,11 +216,14 @@ VQ_DEVINL void scores_tile(float (&s)[NKT][4], const __nv_bfloat16 (*sq)[AT_P], 
   }
   const int q0 = m0 + g + p.q_off;   // absolute position of this thread's first query row (second is q0 + 8)
   if (p.rel_mode == 2) {
-    // bias everywhere (decoder self-attention); rel = key - query is within +-63 by construction
+    // bias everywhere (decoder self-attention); rel = key - query is within +-63 for every row that exists (check_args:
+    // q_off + Sq <= 64). Padded rows (>= Sq, never stored) take the last row's position, so that with a query offset (KV-cache
+    // decoding) their bias index does not leave [0, 127) either.
+    const float* bp0 = sbias + (2 * t - (min(m0 + g, p.Sq - 1) + p.q_off) + (AT_S - 1));
+    const float* bp1 = sbias + (2 * t - (min(m0 + g + 8, p.Sq - 1) + p.q_off) + (AT_S - 1));
 #pragma unroll
     for (int nt = 0; nt < NKT; ++nt) {
-      const float* bp = sbias + (nt * 8 + 2 * t - q0 + (AT_S - 1));
-      s[nt][0] += bp[0]; s[nt][1] += bp[1]; s[nt][2] += bp[-8]; s[nt][3] += bp[-7];
+      s[nt][0] += bp0[nt * 8]; s[nt][1] += bp0[nt * 8 + 1]; s[nt][2] += bp1[nt * 8]; s[nt][3] += bp1[nt * 8 + 1];
     }
   } else if (p.rel_mode == 1 && m0 < p.Lt) {
     // bias on the text x text corner only (encoder): rows / key tiles beyond Lt are skipped warp-uniformly
@@ -536,8 +539,10 @@ VQ_DEVINL void attn_bwd_compute(const AttnArgs& p, const AttnBuckets& bk, const 
   }
   if (NW == 1) __syncwarp(); else __syncthreads();
   // ---- relative-position-bias gradient: d table[bucket(k - q)] += dS[q][k]; one thread per diagonal of the biased
-  //      region sums its <= 64 entries from smem, then one smem atomic per diagonal and one global atomic per bucket ----
-  if (p.d_rel_table) {
+  //      region sums its <= 64 entries from smem, then one smem atomic per diagonal and one global atomic per bucket.
+  //      Without a bias (rel_mode 0) there is no region and the table is left alone. ----
+  const bool d_bias = p.d_rel_table && p.rel_mode;
+  if (d_bias) {
     const int nq = p.rel_mode == 1 ? min(p.Sq, p.Lt) : p.Sq;
     const int nk = p.rel_mode == 1 ? min(p.Sk, p.Lt) : p.Sk;
     const int ndiag = nq + nk - 1;
@@ -579,7 +584,7 @@ VQ_DEVINL void attn_bwd_compute(const AttnArgs& p, const AttnBuckets& bk, const 
     store_tile16(sm.k, m0, dk, p.dk + (size_t)b * p.Sk * p.lddk + h * AT_D, p.lddk, p.Sk, lane);
     store_tile16(sm.v, m0, dv, p.dv + (size_t)b * p.Sk * p.lddv + h * AT_D, p.lddv, p.Sk, lane);
   }
-  if (p.d_rel_table) {
+  if (d_bias) {
     if (NW == 1) __syncwarp(); else __syncthreads();
     for (int i = tid; i < 64; i += NW * 32) {
       const float v = sm.dbucket[i];
@@ -1345,6 +1350,8 @@ static int check_args(const AttnArgs& a) {
     VQ_CHECK(a.rel_mode == 0 || a.Lt <= AT_S, "attention: the biased text x text corner must fit one tile (Lt=%d)", a.Lt);
     VQ_CHECK(!a.q_off, "attention: multi-tile problems take no query offset");
   }
+  VQ_CHECK(a.q_off == 0 || (a.q_off > 0 && a.q_off + a.Sq <= AT_S),
+           "attention: q_off=%d with Sq=%d leaves the %d positions of the relative-position window", a.q_off, a.Sq, AT_S);
   VQ_CHECK(a.ldq % 8 == 0 && a.ldk % 8 == 0 && a.ldv % 8 == 0 && a.ldo % 8 == 0, "attention: pitches must be multiples of 8");
   VQ_CHECK(a.rel_mode == 0 || (a.rel_table && a.rel_bucket), "attention: rel_mode needs rel_table and rel_bucket");
   return 0;

@@ -1162,6 +1162,31 @@ extern "C" int vqacl_attention_bwd(const void* q, const void* k, const void* v, 
   a.o_saved = reinterpret_cast<const bf16*>(o_saved);
   return attn_bwd(a, ST(stream));
 }
+extern "C" int vqacl_attention_fwd_ex(const void* q, const void* k, const void* v, int ldq, int ldk, int ldv, void* o, int ldo,
+                                      float* lse, int B, int H, int Sq, int Sk, const float* rel_table, const int32_t* rel_bucket,
+                                      int rel_mode, int Lt, const float* keymask, int causal, uint32_t drop_thr16, float inv_keep,
+                                      uint32_t drop_key, int64_t q_bstride, int64_t k_bstride, int64_t v_bstride, int64_t o_bstride,
+                                      int q_off, void* stream) {
+  AttnArgs a = make_attn(q, k, v, ldq, ldk, ldv, ldo, lse, B, H, Sq, Sk, rel_table, rel_bucket, rel_mode, Lt, keymask, causal);
+  a.o = reinterpret_cast<bf16*>(o);
+  a.drop_thr = drop_thr16; a.drop_inv_keep = inv_keep; a.seed = drop_key;
+  a.q_bstride = q_bstride; a.k_bstride = k_bstride; a.v_bstride = v_bstride; a.o_bstride = o_bstride; a.q_off = q_off;
+  return attn_fwd(a, ST(stream));
+}
+extern "C" int vqacl_attention_bwd_ex(const void* q, const void* k, const void* v, int ldq, int ldk, int ldv, const void* dO, int ldo,
+                                      const float* lse, void* dq, void* dk, void* dv, int lddq, int lddk, int lddv, int B, int H, int Sq,
+                                      int Sk, const float* rel_table, const int32_t* rel_bucket, int rel_mode, int Lt,
+                                      const float* keymask, int causal, float* d_rel_table, const void* o_saved, uint32_t drop_thr16,
+                                      float inv_keep, uint32_t drop_key, void* stream) {
+  AttnArgs a = make_attn(q, k, v, ldq, ldk, ldv, ldo, const_cast<float*>(lse), B, H, Sq, Sk, rel_table, rel_bucket, rel_mode, Lt,
+                         keymask, causal);
+  a.dO = reinterpret_cast<const bf16*>(dO);
+  a.dq = reinterpret_cast<bf16*>(dq); a.dk = reinterpret_cast<bf16*>(dk); a.dv = reinterpret_cast<bf16*>(dv);
+  a.lddq = lddq; a.lddk = lddk; a.lddv = lddv; a.d_rel_table = d_rel_table;
+  a.o_saved = reinterpret_cast<const bf16*>(o_saved);
+  a.drop_thr = drop_thr16; a.drop_inv_keep = inv_keep; a.seed = drop_key;
+  return attn_bwd(a, ST(stream));
+}
 extern "C" int vqacl_proto_means(const float* h, int B, int S, int split, float* meanQ, float* meanV, void* stream) {
   return proto_means(h, B, S, split, meanQ, meanV, ST(stream));
 }
